@@ -10,6 +10,7 @@ straight into their final bit positions on rank 0 (SURVEY 8(e)).  Weak scaling: 
   value   whole-job MiB/s with the input already resident in HBM when the timed region starts
   e2e     the same through the reference-facing C ABI with a PAGEABLE host buffer (H2D + D2H inside)
   --impl reference   the reference's own CPU implementation (oracle/_ref) on a bounded sample
+  --dump-outputs DIR after the timed steps, the last step's gzip stream as .npy files (see dump_outputs)
 """
 import argparse
 import gzip
@@ -26,6 +27,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import numpy as np  # noqa: E402
+import zref  # noqa: E402
 
 MIB = float(1 << 20)
 MB = 1_000_000               # master block (util.h:60)
@@ -163,18 +165,33 @@ def _ref_part(args):
 
 
 def reference_parts(data, masters, nmasters_total):
-    """ZopfliDeflatePart of sampled master blocks, in a process pool (the children never touch CUDA)"""
+    """ZopfliDeflatePart of sampled master blocks: the reference itself in a process pool (the children never
+    touch CUDA) where oracle/_ref is built, its recorded answers (tests/golden/reference_answers.json) elsewhere"""
     jobs = []
     for m in masters:
         a, b = m * MB, min(len(data), (m + 1) * MB)
         lo = max(0, a - 32768)
         jobs.append((data[lo:b], a - lo, b - lo, int(m == nmasters_total - 1)))
+    if not zref.reference_built(ndebug=True):
+        return zref.reference().map("deflate_part", jobs, numiterations=NUMITER)
     with mp.get_context("fork").Pool(min(8, max(1, len(jobs)))) as pool:
         return pool.map(_ref_part, jobs)
 
 
 def bits_of(b):
     return np.unpackbits(np.frombuffer(b, dtype=np.uint8), bitorder="little")
+
+
+def dump_outputs(path, stream):
+    """The last timed step's result, the gzip stream a caller receives, as float32/float64 .npy files under 64 MB:
+    its length, and its byte values at a fixed seeded sample of at most 4 Mi positions (all of them if shorter)."""
+    os.makedirs(path, exist_ok=True)
+    a = np.frombuffer(stream, dtype=np.uint8)
+    idx = np.arange(len(a)) if len(a) <= (4 << 20) else \
+        np.sort(np.random.default_rng(0).choice(len(a), 4 << 20, replace=False))
+    np.save(os.path.join(path, "gzip_length.npy"), np.array([len(a)], dtype=np.float64))
+    np.save(os.path.join(path, "gzip_sample_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "gzip_sample_bytes.npy"), a[idx].astype(np.float32))
 
 
 def check_against_reference(stream, offs, data, masters, prefix_out=None, prefix_masters=0):
@@ -190,11 +207,10 @@ def check_against_reference(stream, offs, data, masters, prefix_out=None, prefix
         ok &= bool(np.array_equal(body[:n], pb[:n]))
         covered += (prefix_masters - 1) * MB
     want = reference_parts(data, masters, nm)
-    for m, (w, wbp) in zip(masters, want):
-        wb = bits_of(w)
-        nb = int(offs[m + 1] - offs[m])
-        same = nb == len(wb) - ((8 - wbp) & 7) and bool(np.array_equal(body[offs[m]:offs[m + 1]], wb[:nb]))
-        ok &= same
+    for m, w in zip(masters, want):
+        # the master block's bits zero-padded to whole bytes, and its bit count mod 8: ZopfliDeflatePart's (bytes, bp)
+        got = np.packbits(body[offs[m]:offs[m + 1]], bitorder="little").tobytes(), int(offs[m + 1] - offs[m]) & 7
+        ok &= bool(got == w)
         covered += min(len(data), (m + 1) * MB) - m * MB
     return covered, ok
 
@@ -329,16 +345,20 @@ def run_product(args, rank, world):
         nm = (n_total + MB - 1) // MB
         cpu = None
         if world == 1:
-            cpu_v, cpu_sec, ref_out = cpu_reference(data, REF_MASTERS, 1, 0)
-            cpu = {"value": cpu_v, "unit": "MiB/s", "cores": 1, "kind": "reference",
-                   "sample": "first %d bytes (%d master blocks) of the workload, oracle/_ref -O3 -DNDEBUG, 1 thread "
-                             "(the reference has no threading)" % (REF_MASTERS * MB, REF_MASTERS)}
+            ref_out = None   # the CPU baseline needs the reference itself (oracle/_ref), not its recorded answers
+            if zref.reference_built(ndebug=True):
+                cpu_v, cpu_sec, ref_out = cpu_reference(data, REF_MASTERS, 1, 0)
+                cpu = {"value": cpu_v, "unit": "MiB/s", "cores": 1, "kind": "reference",
+                       "sample": "first %d bytes (%d master blocks) of the workload, oracle/_ref -O3 -DNDEBUG, 1 thread "
+                                 "(the reference has no threading)" % (REF_MASTERS * MB, REF_MASTERS)}
             masters = GIANT_MASTERS + UNIFORM_MASTERS if (kind == "synthetic" and WORKLOAD == "c2") else \
                 list(range(REF_MASTERS, nm, max(1, nm // 13)))[:13]
             covered, same = check_against_reference(out_res, offs, data, masters, ref_out, REF_MASTERS)
             check = {"sample_bytes": covered, "identical": bool(same), "delta_bytes_vs_reference": 0 if same else None,
-                     "how": "timed output vs reference: bit prefix of the first %d master blocks + ZopfliDeflatePart of "
-                            "master blocks %s (incl. the five largest blocks), located by bit offsets" % (REF_MASTERS - 1, masters)}
+                     "how": ("timed output vs reference: bit prefix of the first %d master blocks + " % (REF_MASTERS - 1)
+                             if ref_out is not None else "timed output vs the reference's recorded answers: ") +
+                            "ZopfliDeflatePart of master blocks %s (incl. the five largest blocks), located by bit "
+                            "offsets" % masters}
         else:
             # the N-GPU stream must be the single-GPU stream of the same input (itself reference-checked above
             # and in tests/), and sampled master blocks of every rank's shard are compared with the reference
@@ -392,6 +412,8 @@ def run_product(args, rank, world):
                 "output_bytes": len(out_res),
                 "kernel_ms_per_step": {k: v / steps for k, v in st_res.items() if k.startswith("ms_")}}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, out_res)
     if world > 1:
         dist.barrier()
         lib.dist_finalize()
@@ -405,6 +427,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default="c2", help="c2 (default) | c3 (1 GiB, strong scaling) | c4 (binary, 50 iterations)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output there as .npy files")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -25,8 +25,9 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def ref():
+    """the reference's answers (tests/golden/reference_answers.json; the live library while recording)"""
     import zref
-    return zref.Ref()
+    return zref.reference()
 
 
 @pytest.fixture(scope="session")

@@ -34,9 +34,11 @@ def _check(lib_compress, name):
 
 
 @pytest.mark.parametrize("name", sorted(GOLD))
-def test_reference_still_matches_golden(ref, name):
-    """the compiled reference (oracle/_ref) reproduces the committed vectors"""
-    _check(ref.compress, name)
+def test_host_logic_matches_golden(name):
+    """the product's host code over the oracle-backed mock engine (tests/hostmock) reproduces the committed vectors"""
+    import subprocess
+    subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "tests", "hostmock")])
+    _check(zb.Library(os.path.join(ROOT, "tests", "_build", "libzopfli_hostmock.so")).compress, name)
 
 
 @pytest.mark.gpu

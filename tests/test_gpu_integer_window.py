@@ -9,7 +9,6 @@ import sys
 import pytest
 
 import zopfli_b200 as zb
-import zref
 from zopfli_b200 import corpus
 
 pytestmark = pytest.mark.gpu
@@ -23,7 +22,7 @@ CASES = [
 
 
 @pytest.mark.parametrize("name,make,iters", CASES, ids=[c[0] for c in CASES])
-def test_integer_window_runs_and_matches_fp64_and_reference(name, make, iters):
+def test_integer_window_runs_and_matches_fp64_and_reference(ref, name, make, iters):
     data = make()
     lib = zb.library()
     lib.reset_stats()
@@ -32,7 +31,7 @@ def test_integer_window_runs_and_matches_fp64_and_reference(name, make, iters):
     assert st["iterate_steps"] > 0
     if name != "binary":
         assert st["int_steps"] > 0.5 * st["iterate_steps"], "the integer window did not run"
-    assert got == zref.Ref().compress(data, zb.ZOPFLI_FORMAT_DEFLATE, numiterations=iters)
+    assert got == ref.compress(data, zb.ZOPFLI_FORMAT_DEFLATE, numiterations=iters)
     # the same call with the integer window switched off, in a process of its own
     code = ("import sys, hashlib; sys.path.insert(0, %r); import zopfli_b200 as zb; from zopfli_b200 import corpus\n"
             "data = open(sys.argv[1], 'rb').read()\n"

@@ -1,6 +1,5 @@
 """Parity of the sm_100a path (through the C ABI of libzopfli.so.1) against the UNMODIFIED
-reference compiled into oracle/_ref (prebuilt; /root/reference does not exist on the GPU box),
-at the three seams of SURVEY.md section 4.  Integer / byte work: bit-exact, zero tolerance.
+reference's recorded answers (tests/golden/reference_answers.json), at the three seams of SURVEY.md section 4.  Integer / byte work: bit-exact, zero tolerance.
 """
 import zlib
 
@@ -210,7 +209,7 @@ def test_reentrant_concurrent_calls(ref, lib):
     assert got == want
 
 
-def test_verbose_output_matches_reference(tmp_path):
+def test_verbose_output_matches_reference(ref, tmp_path):
     """options.verbose / verbose_more on a one-block input (so the order of the lines is fixed): the
     split-point, per-iteration (squeeze.c:493-495), tree-size and block-size lines on stderr are the
     reference's, byte for byte."""
@@ -235,9 +234,10 @@ a = np.zeros(len(d) + 64, np.uint8); a[:len(d)] = np.frombuffer(d, np.uint8)
 out = C.c_void_p(None); n = C.c_size_t(0)
 lib.ZopfliCompress(C.byref(o), 2, C.c_void_p(a.ctypes.data), C.c_size_t(len(d)), C.byref(out), C.byref(n))
 ''' % (root, os.path.join(root, "tests")))
+
+    def run(which, more):
+        r = subprocess.run([sys.executable, str(script), which, str(more)], capture_output=True, text=True, check=True)
+        return r.stderr.splitlines()
     for more in (0, 1):
-        outs = {}
-        for which in ("ref", "b200"):
-            r = subprocess.run([sys.executable, str(script), which, str(more)], capture_output=True, text=True, check=True)
-            outs[which] = r.stderr.splitlines()
-        assert outs["b200"] == outs["ref"] and any(l.startswith("Iteration") for l in outs["ref"]), more
+        want = ref.answer("verbose_stderr", ("synth_text(120000, 3)", 9, more), lambda r: run("ref", more))
+        assert run("b200", more) == want and any(l.startswith("Iteration") for l in want), more

@@ -1,21 +1,19 @@
-"""Parity with the UNMODIFIED reference (oracle/_ref, prebuilt) at the sizes bench.py runs:
+"""Parity with the UNMODIFIED reference (its recorded answers) at the sizes bench.py runs:
 BASELINE.json configs C2 (100 MB text, 15 iterations) and C4 (51 MB binary, 50 iterations).
 
 The reference needs ~2 s of CPU per master block at 15 iterations, so the full inputs are covered by
 SAMPLED master blocks compared through ZopfliDeflatePart (deflate.c:811-906; a master block is an
 independent unit, deflate.c:908-931): the five master blocks that hold the LARGEST deflate blocks of
 the C2 text (tools/find_giant_masters.py; master 85 holds the 969,128-position block whose DP chain is
-the bench's critical path and whose costs cross 2^21) plus eight uniformly spread ones.  The reference
-side runs in a process pool.  Zero tolerance: byte-identical streams.
+the bench's critical path and whose costs cross 2^21) plus eight uniformly spread ones.  Zero tolerance:
+byte-identical streams.
 """
-import multiprocessing as mp
 import zlib
 
 import numpy as np
 import pytest
 
 import zopfli_b200 as zb
-import zref
 from zopfli_b200 import corpus
 
 pytestmark = pytest.mark.gpu
@@ -27,11 +25,6 @@ GIANT_MASTERS = [85, 84, 78, 42, 40]          # tools/find_giant_masters.py on s
 UNIFORM_MASTERS = [3, 15, 27, 39, 51, 63, 75, 99]
 
 
-def _ref_part(args):
-    piece, s, e, iters, final = args
-    return zref.Ref().deflate_part(piece, s, e, final=final, numiterations=iters)
-
-
 def _slices(data, masters):
     out = []
     for m in masters:
@@ -41,9 +34,8 @@ def _slices(data, masters):
     return out
 
 
-def _reference_parts(parts, iters, final=1):
-    with mp.get_context("fork").Pool(min(8, len(parts))) as pool:  # children never touch CUDA
-        return pool.map(_ref_part, [(p, s, e, iters, final) for p, s, e in parts])
+def _reference_parts(ref, parts, iters, final=1):
+    return ref.map("deflate_part", parts, final=final, numiterations=iters)
 
 
 @pytest.fixture(scope="module")
@@ -56,11 +48,11 @@ def c2():
     return corpus.synth_text(C2_BYTES, 2)
 
 
-def test_c2_giant_and_sampled_master_blocks(lib, c2):
+def test_c2_giant_and_sampled_master_blocks(ref, lib, c2):
     """C2 at 15 iterations: the master blocks holding the five largest blocks + eight sampled ones."""
     masters = GIANT_MASTERS + UNIFORM_MASTERS
     parts = _slices(c2, masters)
-    want = _reference_parts(parts, 15)
+    want = _reference_parts(ref, parts, 15)
     lib.reset_stats()
     for m, (piece, s, e), w in zip(masters, parts, want):
         got = lib.deflate_part(piece, s, e, final=1, numiterations=15)   # (bytes, bp)
@@ -70,7 +62,7 @@ def test_c2_giant_and_sampled_master_blocks(lib, c2):
     assert st["max_block_positions"] >= 900000  # the giant blocks really went through k_iterate
 
 
-def test_c2_whole_stream_contains_the_sampled_master_blocks(lib, c2):
+def test_c2_whole_stream_contains_the_sampled_master_blocks(ref, lib, c2):
     """One ZopfliCompress of the first 45 master blocks (the batched pipelines, lanes and giants of the
     bench) == per-master-block reference spans, compared through the per-master bit offsets."""
     n = 45 * MB
@@ -82,21 +74,20 @@ def test_c2_whole_stream_contains_the_sampled_master_blocks(lib, c2):
     masters = [0, 9, 40, 42, 43]
     parts = _slices(data, masters)
     bits = np.unpackbits(np.frombuffer(z, dtype=np.uint8), bitorder="little")
-    want = _reference_parts(parts, 15, final=0)  # BFINAL is set only on the stream's very last block
-    for m, (w, wbp) in zip(masters, want):
-        wb = np.unpackbits(np.frombuffer(w, dtype=np.uint8), bitorder="little")
-        nb = int(offs[m + 1] - offs[m])
-        assert nb == len(wb) - ((8 - wbp) & 7), (m, nb, len(wb), wbp)
-        assert np.array_equal(bits[offs[m]:offs[m + 1]], wb[:nb]), "master block %d" % m
+    want = _reference_parts(ref, parts, 15, final=0)  # BFINAL is set only on the stream's very last block
+    for m, w in zip(masters, want):
+        # the master block's bits, zero-padded to whole bytes, and its bit count mod 8: (bytes, bp) of ZopfliDeflatePart
+        got = np.packbits(bits[offs[m]:offs[m + 1]], bitorder="little").tobytes(), int(offs[m + 1] - offs[m]) & 7
+        assert got == w, "master block %d" % m
 
 
-def test_c4_binary_50_iterations(lib):
+def test_c4_binary_50_iterations(ref, lib):
     """C4: redundant binary at numiterations=50 -- random restarts + blended statistics
     (squeeze.c:505-517) on full-size master blocks."""
     data = corpus.synth_binary(C4_BYTES, 4)
     masters = [7, 30]
     parts = _slices(data, masters)
-    want = _reference_parts(parts, 50)
+    want = _reference_parts(ref, parts, 50)
     for m, (piece, s, e), w in zip(masters, parts, want):
         got = lib.deflate_part(piece, s, e, final=1, numiterations=50)
         assert got == w, "C4 master block %d differs from the reference" % m
@@ -121,8 +112,8 @@ def test_device_auto_type_bits_seam(ref, lib):
         lo, hi = np.minimum(a, b), np.maximum(a, b)
         lo[0], hi[0] = 0, n
         got = lib.device_auto_type_bits(ll, dd, lo, hi)
-        for i in range(len(lo)):
-            assert float(got[i]) == ref.block_size(data[s:e], ll, dd, int(lo[i]), int(hi[i]), -1), (s, e, lo[i], hi[i])
+        want = ref.many("block_size", [(data[s:e], ll, dd, int(lo[i]), int(hi[i]), -1) for i in range(len(lo))])
+        assert [float(g) for g in got] == want, (s, e)
 
 
 def test_one_block_larger_than_a_master_block(ref, lib):

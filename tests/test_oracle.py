@@ -1,5 +1,5 @@
 """Pins the plain-C restatement (oracle/zopfli_oracle.c) against the UNMODIFIED reference compiled
-from /root/reference (oracle/_ref), at the seams of SURVEY.md section 4:
+from the original project (oracle/_ref; its recorded answers, tests/golden/reference_answers.json), at the seams of SURVEY.md section 4:
   seam 3: per-position ZopfliFindLongestMatch (length, dist, sublen[3..length]) + hash state
   seam 2: ZopfliLZ77Store out of ZopfliLZ77Greedy / ZopfliLZ77Optimal / ZopfliLZ77OptimalFixed
 plus the integer helpers the iterate loop drags in (katajainen.c, tree.c, deflate.c estimators).
@@ -79,6 +79,7 @@ def test_store_seam_50_iterations(ref, oracle):
 
 def test_length_limited_code_lengths(ref, oracle):
     rng = np.random.default_rng(0)
+    calls = []
     for t in range(1500):
         n = int(rng.choice([19, 32, 288]))
         mb = 7 if n == 19 else 15
@@ -96,25 +97,32 @@ def test_length_limited_code_lengths(ref, oracle):
             f[idx] = np.sort(rng.integers(1, 50, k))
         else:  # forces the 15-bit limit with many ties
             f[idx] = (1.5 ** rng.integers(0, 34, k)).astype(np.uint64) + rng.integers(0, 2, k).astype(np.uint64)
-        e1, a = ref.length_limited(f, mb)
+        calls.append((f, mb))
+    for (f, mb), (e1, a) in zip(calls, ref.many("length_limited", calls)):
         e2, b = oracle.length_limited(f, mb)
         assert e1 == e2 and np.array_equal(a, b)
 
 
 def test_entropy_and_rle(ref, oracle):
     rng = np.random.default_rng(1)
+    calls = []
     for t in range(200):
         c = rng.integers(0, 5000, 288).astype(np.uint64)
         c[rng.random(288) < 0.3] = 0
-        assert np.array_equal(ref.entropy(c), oracle.entropy(c))
-    assert np.array_equal(ref.entropy(np.zeros(32)), oracle.entropy(np.zeros(32)))
+        calls.append((c,))
+    calls.append((np.zeros(32),))
+    for (c,), want in zip(calls, ref.many("entropy", calls)):
+        assert np.array_equal(want, oracle.entropy(c))
+    calls = []
     for t in range(400):
         n = int(rng.choice([32, 288]))
         c = rng.integers(0, 30, n).astype(np.uint64)
         c[rng.random(n) < 0.4] = 0
         if t % 3 == 0:
             c = np.repeat(rng.integers(0, 9, n // 8 + 1), 8)[:n].astype(np.uint64)
-        assert np.array_equal(ref.optimize_rle(c), oracle.optimize_rle(c))
+        calls.append((c,))
+    for (c,), want in zip(calls, ref.many("optimize_rle", calls)):
+        assert np.array_equal(want, oracle.optimize_rle(c))
 
 
 # ---- the integer formulation of the forward DP (k_iterate's "integer window", iterate.cuh) ----

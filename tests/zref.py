@@ -1,12 +1,18 @@
 """ctypes bindings used by the tests only.
 
-  ref     -- the UNMODIFIED reference, oracle/_ref/libzopfli_ref.so (+ libref_seams.so wrappers)
-  oracle  -- the plain-C restatement, oracle/_build/libzopfli_oracle.so
+  ref       -- the UNMODIFIED reference, oracle/_ref/libzopfli_ref.so (+ libref_seams.so wrappers)
+  oracle    -- the plain-C restatement, oracle/_build/libzopfli_oracle.so
+  Reference -- the reference's answers to the tests' calls, recorded in tests/golden/reference_answers.json,
+               so that the comparisons run where the reference cannot be built
 Neither is ever imported by the product package.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
+import hashlib
+import json
+import multiprocessing as mp
 import os
 import subprocess
 
@@ -22,13 +28,19 @@ u16p = C.POINTER(C.c_uint16)
 from zopfli_b200 import ZopfliOptions  # same 6-int layout, zopfli.h:33-64
 
 
-def ensure_built():
+def ensure_built(reference=False):
+    """the oracle's libraries; with `reference`, also the reference's (oracle/Makefile builds them where its
+    sources are readable)"""
     need = [os.path.join(ORACLE_DIR, "_build", "libzopfli_oracle.so")]
-    if os.path.isdir("/root/reference/src/zopfli"):
+    if reference:
         need += [os.path.join(ORACLE_DIR, "_ref", "libzopfli_ref.so"),
                  os.path.join(ORACLE_DIR, "_ref", "libref_seams.so")]
     if not all(os.path.exists(p) for p in need):
-        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "all"])
+        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "all" if reference else "oracle"])
+
+
+def reference_built(ndebug=False):
+    return os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libzopfli_ref_ndebug.so" if ndebug else "libzopfli_ref.so"))
 
 
 def _np_u8(b):
@@ -45,7 +57,7 @@ def _ptr(a, t):
 
 class Ref:
     def __init__(self, ndebug=False):
-        ensure_built()
+        ensure_built(reference=True)
         name = "libzopfli_ref_ndebug.so" if ndebug else "libzopfli_ref.so"
         self.lib = C.CDLL(os.path.join(ORACLE_DIR, "_ref", name))
         self.seams = C.CDLL(os.path.join(ORACLE_DIR, "_ref", "libref_seams.so"))
@@ -330,3 +342,192 @@ def histogram(litlens, dists):
     ds[big] = 2 * l + ((x >> (l - 1)) & 1)
     dc = np.bincount(ds, minlength=32)[:32].astype(np.uint64)
     return llc, dc
+
+
+# ---- the reference's answers, recorded ----
+# The reference cannot be built everywhere the tests run (its sources are not part of this repository), so every
+# call the tests make to it is answered from tests/golden/reference_answers.json.  Small answers are stored as
+# they are; bytes and arrays longer than VERBATIM by length and SHA-256.  Where the oracle restatement computes
+# the same function, a digest-only answer is the oracle's value after checking it against the digest, so the
+# tests can keep using reference parses as inputs.  To record (where oracle/_ref is built):
+#   ZOPFLI_B200_RECORD_REFERENCE=tests/golden/reference_answers.json python -m pytest tests ...
+ANSWERS = os.path.join(ROOT, "tests", "golden", "reference_answers.json")
+VERBATIM = 64
+ORACLE_EQUIVALENT = ("lz77", "match_table", "limited_match", "length_limited", "entropy", "optimize_rle")
+REF_METHODS = ORACLE_EQUIVALENT + ("compress", "deflate_part", "block_size", "block_split_lz77", "block_split")
+
+
+def _sha(b):
+    return hashlib.sha256(b).hexdigest()
+
+
+def encode(x, digest=False):
+    """JSON form of a value: small bytes / arrays as they are (unless `digest`), larger ones by digest"""
+    if isinstance(x, (bytes, bytearray, memoryview)):
+        x = bytes(x)
+        return {"hex": x.hex()} if len(x) <= VERBATIM and not digest else {"bytes": len(x), "sha256": _sha(x)}
+    if isinstance(x, np.ndarray):
+        a = np.ascontiguousarray(x)
+        if a.size <= VERBATIM and not digest:
+            return {"dtype": a.dtype.str, "shape": list(a.shape), "data": a.tolist()}
+        return {"dtype": a.dtype.str, "shape": list(a.shape), "sha256": _sha(a.tobytes())}
+    if isinstance(x, tuple):
+        return {"tuple": [encode(v, digest) for v in x]}
+    if isinstance(x, list):
+        return [encode(v, digest) for v in x]
+    if isinstance(x, dict):
+        return {"kw": {k: encode(v, digest) for k, v in sorted(x.items())}}
+    if isinstance(x, np.integer):
+        return int(x)
+    if isinstance(x, np.floating):
+        return float(x)
+    return x
+
+
+def _list_digest(values):
+    return {"items": len(values), "sha256": _sha(json.dumps(encode(values, True), sort_keys=True).encode())}
+
+
+class Recorded:
+    """An answer of the reference known by its digest: equal to any value with the same digest."""
+
+    def __init__(self, rec):
+        self.rec = rec
+
+    def __eq__(self, other):
+        if "items" in self.rec:
+            return isinstance(other, list) and _list_digest(other) == self.rec
+        return encode(other, True) == self.rec
+
+    def __len__(self):
+        return self.rec["items"] if "items" in self.rec else self.rec["bytes"]
+
+    def __repr__(self):
+        return "<reference answer %s>" % json.dumps(self.rec)
+
+
+def _decode(rec, computed=None, what=""):
+    if isinstance(rec, list):
+        return [_decode(r, None if computed is None else c, what) for r, c in
+                zip(rec, computed if computed is not None else [None] * len(rec))]
+    if not isinstance(rec, dict):
+        return rec
+    if "tuple" in rec:
+        cs = computed if computed is not None else [None] * len(rec["tuple"])
+        return tuple(_decode(r, c, what) for r, c in zip(rec["tuple"], cs))
+    if "hex" in rec:
+        return bytes.fromhex(rec["hex"])
+    if "data" in rec:
+        return np.array(rec["data"], dtype=np.dtype(rec["dtype"])).reshape(rec["shape"])
+    if computed is None:
+        return Recorded(rec)
+    assert encode(computed, True) == rec, "the oracle restatement's %s differs from the reference's" % what
+    return computed
+
+
+def _live_call(args):
+    method, a, kw = args
+    return getattr(Ref(), method)(*a, **kw)
+
+
+class Reference:
+    """The reference's answers with the methods of `Ref`: recorded ones by default, the live library while
+    recording (ZOPFLI_B200_RECORD_REFERENCE=<file>: the answers file plus the new answers is written there)."""
+
+    def __init__(self):
+        self.out = os.environ.get("ZOPFLI_B200_RECORD_REFERENCE")
+        self.live = Ref() if self.out else None
+        self.table = json.load(open(ANSWERS)) if os.path.exists(ANSWERS) else {}
+        self._oracle = None
+        if self.out:
+            if os.path.exists(self.out):   # successive recording processes add to one file
+                self.table.update(json.load(open(self.out)))
+            atexit.register(self.save)
+
+    def save(self):
+        with open(self.out, "w") as f:
+            f.write("{\n" + ",\n".join(json.dumps(k) + ": " + json.dumps(self.table[k], sort_keys=True, separators=(",", ":"))
+                                      for k in sorted(self.table)) + "\n}\n")
+
+    @property
+    def oracle(self):
+        if self._oracle is None:
+            self._oracle = Oracle()
+        return self._oracle
+
+    @staticmethod
+    def _key(method, args, kw):
+        return method + ":" + _sha(json.dumps(encode((args, kw), True), sort_keys=True).encode())[:32]
+
+    def _lookup(self, key):
+        assert key in self.table, "no recorded reference answer for %s: record it where oracle/_ref is built" % key
+        return self.table[key]
+
+    def call(self, method, *args, **kw):
+        key = self._key(method, args, kw)
+        if self.live is not None:
+            value = getattr(self.live, method)(*args, **kw)
+            self.table[key] = encode(value)
+            return value
+        rec = self._lookup(key)
+        computed = getattr(self.oracle, method)(*args, **kw) if method in ORACLE_EQUIVALENT and \
+            _needs_digest_check(rec) else None
+        return _decode(rec, computed, method)
+
+    def many(self, method, calls):
+        """[method(*c) for c in calls], recorded as one digest"""
+        key = self._key("many/" + method, calls, {})
+        if self.live is not None:
+            values = [getattr(self.live, method)(*c) for c in calls]
+            self.table[key] = _list_digest(values)
+            return values
+        rec = self._lookup(key)
+        if method not in ORACLE_EQUIVALENT:
+            return Recorded(rec)
+        values = [getattr(self.oracle, method)(*c) for c in calls]
+        assert _list_digest(values) == rec, "the oracle restatement's %s differs from the reference's" % method
+        return values
+
+    def map(self, method, calls, **kw):
+        """[method(*c, **kw) for c in calls]: while recording in a process pool (the children never touch CUDA)"""
+        if self.live is None:
+            return [self.call(method, *c, **kw) for c in calls]
+        with mp.get_context("fork").Pool(min(8, max(1, len(calls)))) as pool:
+            values = pool.map(_live_call, [(method, c, kw) for c in calls])
+        for c, v in zip(calls, values):
+            self.table[self._key(method, c, kw)] = encode(v)
+        return values
+
+    def answer(self, name, args, live, digest=False):
+        """an answer that needs more than one call: live(ref) computes it from the `Ref` library"""
+        key = self._key(name, args, {})
+        if self.live is not None:
+            value = live(self.live)
+            self.table[key] = _list_digest(value) if digest else encode(value)
+            return value
+        return _decode(self._lookup(key))
+
+    def __getattr__(self, method):
+        if method not in REF_METHODS:
+            raise AttributeError(method)
+        return lambda *a, **kw: self.call(method, *a, **kw)
+
+
+def _needs_digest_check(rec):
+    if isinstance(rec, list):
+        return any(_needs_digest_check(r) for r in rec)
+    if isinstance(rec, dict):
+        if "tuple" in rec:
+            return any(_needs_digest_check(r) for r in rec["tuple"])
+        return "sha256" in rec
+    return False
+
+
+_reference = None
+
+
+def reference() -> Reference:
+    global _reference
+    if _reference is None:
+        _reference = Reference()
+    return _reference
